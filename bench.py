@@ -4,6 +4,7 @@ atom-updates/sec per MD step, SevenNet-0, 1/2/4/8 B200).
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA engine
     python bench.py --impl reference --gpus N --steps K ...   # the CPU oracle (reference arm)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's results as DIR/*.npy
 
 One "step" = one energy+force evaluation of one periodic Si cell with a fixed neighbour list:
   N = 1 : BASELINE configs[1], SevenNet-0, Si 10x10x15 = 12 000 atoms, 336 000 edges
@@ -79,6 +80,45 @@ class ClockSampler:
                 'samples': len(sm), 'reasons': sorted(reasons)}
 
 
+DUMP_LIMIT = 60 << 20      # bytes of array data written by --dump-outputs (the .npy headers stay within 64 MB)
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """--dump-outputs: every array as <out_dir>/<name>.npy in float32 or float64, so that two builds of the project
+    can be compared output by output on identical inputs.  Should the arrays exceed `limit` bytes in all, the largest
+    keep a fixed sample of their rows (RandomState(0), sorted): the same rows for the same shapes."""
+    arrs = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, 'detach') else np.asarray(a)
+        arrs[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    left = limit
+    for i, name in enumerate(sorted(arrs, key=lambda k: arrs[k].nbytes)):
+        a = arrs[name]
+        share = left // (len(arrs) - i)
+        if a.nbytes > share:
+            rows = np.random.RandomState(0).choice(len(a), share // (a.nbytes // len(a)), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, f'{name}.npy'), a)
+        left -= a.nbytes
+    print(f'bench: wrote {", ".join(sorted(arrs))} to {out_dir}', file=sys.stderr, flush=True)
+
+
+def global_results(r, n_global, dev):
+    """the distributed runner's per-rank results -> energy, virial and per-atom arrays over all atoms in the global
+    atom order, on every rank (collective)"""
+    import torch
+    import torch.distributed as dist
+    gids = torch.as_tensor(np.asarray(r['global_ids']), dtype=torch.long, device=dev)
+    out = {'energy': r['energy'], 'virial': r['virial']}
+    for k in ('atomic_energy', 'forces'):
+        full = torch.zeros((n_global,) + tuple(r[k].shape[1:]), dtype=r[k].dtype, device=dev)
+        full[gids] = r[k]
+        dist.all_reduce(full)
+        out[k] = full
+    return out
+
+
 def make_system(cells):
     from sevenn_b200.neighbors import build_graph, diamond_si
     pos, cell, z = diamond_si(*cells)
@@ -142,8 +182,10 @@ def run_reference(args):
     times = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        o.forward(sp, ei, ev)
+        out = o.forward(sp, ei, ev)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v for k, v in out.items() if isinstance(v, torch.Tensor) and v.is_floating_point()})
     total = sum(times)
     value = n_atoms * args.steps / total
     line = {
@@ -347,6 +389,12 @@ def run_engine(args):
         runner.set_cuda_graph(True)
     total_ms, launches, clocks = timed_run()
     value = n_atoms * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs:       # the last timed step's results, read before any later leg runs the engine again
+        res = (runner or eng).results()
+        if world > 1:
+            res = global_results(res, n_atoms, dev)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, res)
 
     # ---- per-kernel breakdown + roofline of the dominant kernel (rank 0) ---------------------------
     # (every rank runs the same steps -- the exchanges are collective; only rank 0 records events)
@@ -639,6 +687,13 @@ def run_nacl_d3(args):
         t_d3 += b.elapsed_time(c)
     clocks = sampler.stop()
     launches = (eng if world == 1 else runner).launch_count()      # network kernels only (the D3 library entry points do not feed this counter)
+    if args.dump_outputs:
+        res = (eng if world == 1 else runner).results()
+        if world > 1:
+            res = global_results(res, n_atoms, dev)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {**{f'network_{k}': v for k, v in res.items()},
+                                             'd3_energy': np.float64(e_d3), 'd3_forces': f_d3, 'd3_sigma': s_d3})
     tt = torch.tensor([total, t_net, t_d3], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -786,9 +841,14 @@ def main():
                     help="'si': the headline benchmark (BASELINE configs[1]/[3]); 'nacl_d3': configs[4], SevenNet-0 + D3 on NaCl")
     ap.add_argument('--nacl-a', type=float, default=5.64,
                     help='lattice constant of the nacl_d3 workload; 4.0 is the dense variant of SURVEY 8(d).5 (about 65 neighbours per atom)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the results of the last one as DIR/<name>.npy (float32/float64, '
+                         'at most 64 MB in all); the inputs are the same on every run with the same arguments')
     args = ap.parse_args()
     if args.gpus not in CELLS:
         raise SystemExit('--gpus must be 1, 2, 4 or 8')
+    if args.steps < 1:
+        raise SystemExit('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     elif args.workload == 'nacl_d3':

@@ -1,6 +1,8 @@
 """GPU parity of the cell-list D3 kernels (csrc/d3_kernels.cuh through the C ABI) against the fp64 oracle
-(oracle/d3_oracle.py) and the reference's golden values (tests/unit_tests/test_calculator.py:192-238)."""
+(oracle/d3_oracle.py), the reference's golden values (tests/unit_tests/test_calculator.py:192-238) and the stored
+results of the reference's own CUDA D3 (tests/golden/d3_reference_nacl.npz)."""
 import ctypes
+import os
 
 import numpy as np
 import pytest
@@ -100,55 +102,16 @@ def test_reference_named_entry_points():
     assert _rel(s, [sg[0, 0], sg[1, 1], sg[2, 2], sg[0, 1], sg[0, 2], sg[1, 2]]) < 2e-5
 
 
-def _reference_lib():
-    import os
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', 'oracle', '_ref', 'libpaird3.so')
-    if not os.path.exists(path):
-        pytest.skip('oracle/_ref/libpaird3.so not built (make -C oracle, needs /root/reference)')
-    lib = ctypes.CDLL(path)
-    lib.pair_init.restype = ctypes.c_void_p
-    lib.pair_get_energy.restype = ctypes.c_double
-    lib.pair_get_force.restype = ctypes.POINTER(ctypes.c_double)
-    lib.pair_get_stress.restype = ctypes.POINTER(ctypes.c_double * 6)
-    for fn in ('pair_set_atom', 'pair_set_domain', 'pair_run_settings', 'pair_run_coeff', 'pair_run_compute', 'pair_fin'):
-        getattr(lib, fn).restype = None
-    lib.pair_get_energy.argtypes = lib.pair_get_force.argtypes = lib.pair_get_stress.argtypes = [ctypes.c_void_p]
-    lib.pair_set_atom.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
-    lib.pair_set_domain.argtypes = [ctypes.c_void_p] + [ctypes.c_int] * 3 + [ctypes.c_void_p] * 2 + [ctypes.c_double] * 3
-    lib.pair_run_settings.argtypes = [ctypes.c_void_p, ctypes.c_double, ctypes.c_double, ctypes.c_char_p, ctypes.c_char_p]
-    lib.pair_run_coeff.argtypes = [ctypes.c_void_p, ctypes.c_void_p]
-    lib.pair_run_compute.argtypes = lib.pair_fin.argtypes = [ctypes.c_void_p]
-    return lib
-
-
-def run_reference_d3(lib, z, pos, cell, damping=b'damp_bj'):
-    """the compiled, unmodified reference (orthogonal / lower-triangular cells only: no frame rotation here)"""
-    uniq = list(dict.fromkeys(np.asarray(z).tolist()))
-    types = np.ascontiguousarray([uniq.index(a) + 1 for a in z], dtype=np.int32)
-    x = np.ascontiguousarray(pos, dtype=np.float64)
-    nums = np.ascontiguousarray(uniq, dtype=np.int32)
-    lo, hi = np.zeros(3), np.ascontiguousarray([cell[0, 0], cell[1, 1], cell[2, 2]], dtype=np.float64)
-    p = lib.pair_init()
-    lib.pair_set_atom(p, len(z), len(uniq), types.ctypes.data, x.ctypes.data)
-    lib.pair_set_domain(p, 1, 1, 1, lo.ctypes.data, hi.ctypes.data, float(cell[1, 0]), float(cell[2, 0]), float(cell[2, 1]))
-    lib.pair_run_settings(p, 9000.0, 1600.0, damping, b'pbe')
-    lib.pair_run_coeff(p, nums.ctypes.data)
-    lib.pair_run_compute(p)
-    e = lib.pair_get_energy(p)
-    f = np.ctypeslib.as_array(lib.pair_get_force(p), shape=(len(z) * 3,)).reshape(-1, 3).copy()
-    s = np.array(lib.pair_get_stress(p).contents)
-    return e, f, s
-
-
 @pytest.mark.parametrize('cells,damping', [((2, 2, 2), 'damp_bj'), ((6, 6, 4), 'damp_bj'), ((5, 5, 5), 'damp_zero')])
 def test_matches_compiled_reference(cells, damping):
-    """oracle/_ref = the reference's own CUDA D3, default cutoffs, rocksalt NaCl (64 / 1152 / 1000 atoms).  The
-    reference sums its lattice images in fp32 (see tests/test_d3_oracle.py), hence 1e-4 on the energy."""
+    """The reference's own CUDA D3 at its default cutoffs on rocksalt NaCl (64 / 1152 / 1000 atoms): inputs and
+    results stored in tests/golden/d3_reference_nacl.npz by tools/make_d3_golden.py.  The reference sums its
+    lattice images in fp32 (see tests/test_d3_oracle.py), hence 1e-4 on the energy."""
     from sevenn_b200.d3 import D3Engine
-    from sevenn_b200.neighbors import rocksalt_nacl
-    lib = _reference_lib()
-    pos, cell, z = rocksalt_nacl(*cells, sigma=0.05, seed=11)
-    e_ref, f_ref, s_ref = run_reference_d3(lib, z, pos, cell, damping.encode())
+    key = 'nacl_{}x{}x{}_{}'.format(*cells, damping)
+    with np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'd3_reference_nacl.npz')) as g:
+        z, pos, cell = g[f'{key}_numbers'], g[f'{key}_positions'], g[f'{key}_cell']
+        e_ref, f_ref, s_ref = float(g[f'{key}_energy']), g[f'{key}_forces'], g[f'{key}_sigma']
     e, f, s = D3Engine(damping, 'pbe').compute(z, pos, cell)
     assert abs(e / e_ref - 1.0) < 1e-4
     assert np.abs(f - f_ref).max() < 2e-6 + 1e-4 * np.abs(f_ref).max()

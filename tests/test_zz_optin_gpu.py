@@ -112,7 +112,12 @@ def test_gate_bwd_rows_option_matches_default(model):
         out = {k: v.cpu().numpy().copy() for k, v in eng.results().items()}
     finally:
         set_option('gate_bwd_rows', 0)
-    assert out['energy'][0] == ref['energy'][0]
+    # the option changes the backward only: every per-atom energy is bit-identical; the total is a double atomicAdd of
+    # per-block partial sums (readout_kernel) in an order that varies from run to run, so it is equal up to the
+    # rounding of a reordered sum of n terms
+    assert np.array_equal(out['atomic_energy'], ref['atomic_energy'])
+    n = len(ref['atomic_energy'])
+    assert abs(out['energy'][0] - ref['energy'][0]) <= n * np.finfo(np.float64).eps * np.abs(ref['atomic_energy']).sum()
     assert np.allclose(out['forces'], ref['forces'], atol=2e-6)
     assert np.allclose(out['virial'], ref['virial'], atol=1e-5)
 

@@ -3,8 +3,8 @@
 
 Evidence for which hardware paths each kernel uses (B200_PROFILING.md, "What proves a Blackwell-native
 kernel"): UTC*MMA = tcgen05.mma, LDTM/STTM = tcgen05.ld/st, UTMALDG/UTMASTG = TMA tensor copies,
-UBLKCP = cp.async.bulk, FFMA2/FMUL2 = packed fp32, RED/ATOM = reductions.  Regenerated by
-__graft_entry__.build(); runs on the CPU box (cuobjdump needs no GPU)."""
+UBLKCP = cp.async.bulk, FFMA2/FMUL2 = packed fp32, RED/ATOM = reductions.  __graft_entry__.build() writes
+the same summary to sevenn_b200/csrc/build/sass_summary.txt; runs without a GPU (cuobjdump needs none)."""
 import collections
 import os
 import re
