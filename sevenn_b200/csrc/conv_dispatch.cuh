@@ -3,21 +3,13 @@
 #pragma once
 #include "conv_kernels.cuh"
 
-#ifndef S7B_BWD_L0_NV
-#define S7B_BWD_L0_NV 2   // channel pairs per lane in the l1 = 0 backward kernels (1 is 6% faster but splits a
-                          // (node, l1) role over two CTAs, whose per-edge dY/dE/dr sums then need atomics)
-#endif
-
-#ifndef S7B_FWD_L0_NV
-#define S7B_FWD_L0_NV 2   // channel pairs per lane in the l1 = 0 forward kernels (1 was measured 4 % slower)
-#endif
-#ifndef S7B_FWD_ODD_PAIRS
-#define S7B_FWD_ODD_PAIRS 1   // mul = 32 forward kernels: 1 = channel pairs on half warps (two nodes per warp, FFMA2),
-                              // 0 = one channel per lane.  Pairs are 29 % faster since the edge records are fetched
-                              // cooperatively (0.099 vs 0.139 ms, 7net-0 l1 = 2); before that the scalar form won.
-#endif
-
 namespace s7b {
+
+// channel pairs per lane in the l1 = 0 backward kernels (1 is 6% faster but splits a (node, l1) role over
+// two CTAs, whose per-edge dY/dE/dr sums then need atomics)
+constexpr int kBwdL0NV = 2;
+// channel pairs per lane in the l1 = 0 forward kernels (1 was measured 4 % slower)
+constexpr int kFwdL0NV = 2;
 
 template <int LPN>
 static inline dim3 conv_grid(const ConvArgs& a, const ConvRole& role, int nv) {
@@ -28,17 +20,8 @@ static inline dim3 conv_grid(const ConvArgs& a, const ConvRole& role, int nv) {
 template <class Kind, int NV, int LPN>
 static int launch_fwd_one(bool table, const ConvArgs& a, const ConvRole& role, float* out, cudaStream_t st) {
   const dim3 grid = conv_grid<LPN>(a, role, NV);
-  if (table) conv_fwd_kernel<Kind, NV, LPN, true, V2><<<grid, 32 * kConvWarpsPerBlock, 0, st>>>(a, role, out);
-  else conv_fwd_kernel<Kind, NV, LPN, false, V2><<<grid, 32 * kConvWarpsPerBlock, 0, st>>>(a, role, out);
-  return cudaGetLastError() == cudaSuccess ? 0 : 1;
-}
-
-// one channel per lane, a full warp per node (alternative forward mapping for mul = 32, see S7B_FWD_ODD_PAIRS)
-template <class Kind>
-static int launch_fwd_scalar(bool table, const ConvArgs& a, const ConvRole& role, float* out, cudaStream_t st) {
-  dim3 grid((a.n_dst - a.n_begin + kConvWarpsPerBlock - 1) / kConvWarpsPerBlock, role.mul / 32);
-  if (table) conv_fwd_kernel<Kind, 1, 32, true, float><<<grid, 32 * kConvWarpsPerBlock, 0, st>>>(a, role, out);
-  else conv_fwd_kernel<Kind, 1, 32, false, float><<<grid, 32 * kConvWarpsPerBlock, 0, st>>>(a, role, out);
+  if (table) conv_fwd_kernel<Kind, NV, LPN, true><<<grid, 32 * kConvWarpsPerBlock, 0, st>>>(a, role, out);
+  else conv_fwd_kernel<Kind, NV, LPN, false><<<grid, 32 * kConvWarpsPerBlock, 0, st>>>(a, role, out);
   return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 
@@ -66,16 +49,13 @@ static int launch_bwd_one(bool table, bool need_dx, const ConvArgs& a, const Con
 }
 
 // Lane mapping by multiplicity: 128 | mul -> a warp per node, 2 channel pairs per lane (only
-// instantiated where MAXNV == 2); 64 | mul -> a warp per node, 1 pair; else half a warp per node.
+// instantiated where MAXNV == 2); 64 | mul -> a warp per node, 1 pair; else half a warp per node
+// (for mul = 32, 29 % faster than one channel per lane on a full warp: 0.099 vs 0.139 ms, 7net-0 l1 = 2).
 template <class Kind, int MAXNV>
 static int fwd_kind(bool table, const ConvArgs& a, const ConvRole& role, float* out, cudaStream_t st) {
   if (MAXNV >= 2 && role.mul % 128 == 0) return launch_fwd_one<Kind, MAXNV, 32>(table, a, role, out, st);
   if (role.mul % 64 == 0) return launch_fwd_one<Kind, 1, 32>(table, a, role, out, st);
-#if S7B_FWD_ODD_PAIRS
   return launch_fwd_one<Kind, 1, 16>(table, a, role, out, st);
-#else
-  return launch_fwd_scalar<Kind>(table, a, role, out, st);
-#endif
 }
 
 // ALLOW_NODX: only the l1 = 0 kinds are ever run without dx (first layer: x depends on species only)
@@ -97,7 +77,7 @@ static int bwd_kind(bool table, bool need_dx, const ConvArgs& a, const ConvRole&
   int launch_conv_fwd_##LF##_##LO(int l1, bool table, const ConvArgs& a, const ConvRole& role,     \
                                   float* out, cudaStream_t st) {                                   \
     switch (l1) {                                                                                  \
-      case 0: return fwd_kind<TPKind<0, LF, LO>, S7B_FWD_L0_NV>(table, a, role, out, st);                      \
+      case 0: return fwd_kind<TPKind<0, LF, LO>, kFwdL0NV>(table, a, role, out, st);                      \
       case 1: return fwd_kind<TPKind<1, LF, LO>, 1>(table, a, role, out, st);                      \
       case 2: return fwd_kind<TPKind<2, LF, LO>, 1>(table, a, role, out, st);                      \
       case 3: return fwd_kind<TPKind<(LF >= 3 ? 3 : 2), LF, LO>, 1>(table, a, role, out, st);      \
@@ -108,7 +88,7 @@ static int bwd_kind(bool table, bool need_dx, const ConvArgs& a, const ConvRole&
                                   const ConvRole& role, const float* gout, float* dx, float* dY,   \
                                   float* dEdr, float* dw, cudaStream_t st) {                       \
     switch (l1) {                                                                                  \
-      case 0: return bwd_kind<TPKind<0, LF, LO>, S7B_BWD_L0_NV, true>(table, need_dx, a, role, gout, dx, dY, dEdr, dw, st);  \
+      case 0: return bwd_kind<TPKind<0, LF, LO>, kBwdL0NV, true>(table, need_dx, a, role, gout, dx, dY, dEdr, dw, st);  \
       case 1: return bwd_kind<TPKind<1, LF, LO>, 1, false>(table, need_dx, a, role, gout, dx, dY, dEdr, dw, st); \
       case 2: return bwd_kind<TPKind<2, LF, LO>, 1, false>(table, need_dx, a, role, gout, dx, dY, dEdr, dw, st); \
       case 3: return bwd_kind<TPKind<(LF >= 3 ? 3 : 2), LF, LO>, 1, false>(table, need_dx, a, role, gout, dx, dY, dEdr, dw, st); \

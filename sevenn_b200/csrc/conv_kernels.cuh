@@ -33,18 +33,8 @@ constexpr int kConvWarpsPerBlock = 4;
 //  * backward: l1 = 0 is fastest at 3 (-6 %), l1 = 1 at 4 (128 registers; 168 or 220 are 3-4 % slower),
 //    l1 >= 2 at 3 (what ptxas picks by itself).  The lmax = 3 kinds need > 168 registers (they spill
 //    otherwise) and are left at 2.
-#ifndef S7B_FWD_MINBLOCKS
-#define S7B_FWD_MINBLOCKS 1
-#endif
-#define S7B_FWD_BOUNDS __launch_bounds__(32 * kConvWarpsPerBlock, S7B_FWD_MINBLOCKS)
-#ifdef S7B_BWD_MINBLOCKS
-#define S7B_BWD_BOUNDS __launch_bounds__(32 * kConvWarpsPerBlock, S7B_BWD_MINBLOCKS)
-#else
+#define S7B_FWD_BOUNDS __launch_bounds__(32 * kConvWarpsPerBlock, 1)
 #define S7B_BWD_BOUNDS __launch_bounds__(32 * kConvWarpsPerBlock, (Kind::NY != 9) ? 2 : ((Kind::D1 == 3) ? 4 : 3))
-#endif
-#ifndef S7B_COOP_REC
-#define S7B_COOP_REC 1   // lanes of a group fetch the records of LPN consecutive edges at once (see EdgeRecs)
-#endif
 
 // The 16-byte edge record {neighbour, table interval, frac} heads the per-edge dependency chain
 // (record -> gather address / table address -> loads -> math).  Loading it per edge costs one
@@ -112,49 +102,19 @@ __device__ __forceinline__ void load_Y(const float* __restrict__ Yrow, float (&Y
 
 __device__ __forceinline__ float2 ldg2(const float* p) { return __ldg(reinterpret_cast<const float2*>(p)); }
 
-// Per-lane value type: V2 = two adjacent channels (packed FFMA2 math), float = one channel.
-template <class V> struct VT;
-template <> struct VT<V2> {
-  static constexpr int CH = 2;
-  static __device__ __forceinline__ V2 zero() { return splat2(0.0f); }
-  static __device__ __forceinline__ V2 load(const float* p) { return ldg2(p); }
-  static __device__ __forceinline__ void store(float* p, V2 v) { *reinterpret_cast<float2*>(p) = v; }
-  static __device__ __forceinline__ float hsum(V2 v) { return v.x + v.y; }
-  static __device__ __forceinline__ float amax(V2 v) { return fmaxf(fabsf(v.x), fabsf(v.y)); }
-  // cubic coefficients of the channel pair starting at (even) column c of table row tk
-  static __device__ __forceinline__ void coef(const ConvArgs& a, int tk, int c, V2& a0, V2& a1, V2& a2, V2& a3) {
-    const size_t ti = (size_t)tk * (a.w_numel >> 1) + (c >> 1);
-    const float4 c01 = __ldg(a.table + ti);
-    const uint2 c23 = __ldg(a.table23 + ti);
-    a0 = make_float2(c01.x, c01.y);
-    a1 = make_float2(c01.z, c01.w);
-    a2 = __half22float2(*reinterpret_cast<const __half2*>(&c23.x));
-    a3 = __half22float2(*reinterpret_cast<const __half2*>(&c23.y));
-  }
-};
-template <> struct VT<float> {
-  static constexpr int CH = 1;
-  static __device__ __forceinline__ float zero() { return 0.0f; }
-  static __device__ __forceinline__ float load(const float* p) { return __ldg(p); }
-  static __device__ __forceinline__ void store(float* p, float v) { *p = v; }
-  static __device__ __forceinline__ float hsum(float v) { return v; }
-  static __device__ __forceinline__ float amax(float v) { return fabsf(v); }
-  static __device__ __forceinline__ void coef(const ConvArgs& a, int tk, int c, float& a0, float& a1, float& a2, float& a3) {
-    const size_t ti = (size_t)tk * (a.w_numel >> 1) + (c >> 1);
-    const float4 c01 = __ldg(a.table + ti);
-    const uint2 c23 = __ldg(a.table23 + ti);
-    const float2 h2 = __half22float2(*reinterpret_cast<const __half2*>(&c23.x));
-    const float2 h3 = __half22float2(*reinterpret_cast<const __half2*>(&c23.y));
-    const bool odd = (c & 1) != 0;
-    a0 = odd ? c01.y : c01.x;
-    a1 = odd ? c01.w : c01.z;
-    a2 = odd ? h2.y : h2.x;
-    a3 = odd ? h3.y : h3.x;
-  }
-};
+// cubic coefficients of the channel pair starting at (even) column c of table row tk
+__device__ __forceinline__ void table_coef(const ConvArgs& a, int tk, int c, V2& a0, V2& a1, V2& a2, V2& a3) {
+  const size_t ti = (size_t)tk * (a.w_numel >> 1) + (c >> 1);
+  const float4 c01 = __ldg(a.table + ti);
+  const uint2 c23 = __ldg(a.table23 + ti);
+  a0 = make_float2(c01.x, c01.y);
+  a1 = make_float2(c01.z, c01.w);
+  a2 = __half22float2(*reinterpret_cast<const __half2*>(&c23.x));
+  a3 = __half22float2(*reinterpret_cast<const __half2*>(&c23.y));
+}
 
 // Which node / channel pair this lane works on.
-template <int NV, int LPN, int CH>
+template <int NV, int LPN>
 struct LaneMap {
   int n, sl, uc0, e0, len, nmax;
   bool node_ok;
@@ -164,7 +124,7 @@ struct LaneMap {
     sl = lane % LPN;
     n = a.n_begin + (blockIdx.x * kConvWarpsPerBlock + (threadIdx.x >> 5)) * GPW + lane / LPN;
     node_ok = n < a.n_dst;
-    uc0 = blockIdx.y * (CH * LPN * NV) + CH * sl;
+    uc0 = blockIdx.y * (2 * LPN * NV) + 2 * sl;
     e0 = 0;
     len = 0;
     if (node_ok) {
@@ -180,49 +140,44 @@ struct LaneMap {
 // forward:  out[n, path block] = sum_{e in row n} w_e * CG(x[src_e], Y_e)
 // grid = (ceil(n_dst / (kConvWarpsPerBlock * 32/LPN)), mul / (2*LPN*NV)), block = 32*kConvWarpsPerBlock
 // ------------------------------------------------------------------------------------------
-template <class Kind, int NV, int LPN, bool TABLE, class V>
+template <class Kind, int NV, int LPN, bool TABLE>
 __global__ void S7B_FWD_BOUNDS
 conv_fwd_kernel(const ConvArgs a, const ConvRole role, float* __restrict__ out) {
-  constexpr int CH = VT<V>::CH;
-  const LaneMap<NV, LPN, CH> m(a);
+  const LaneMap<NV, LPN> m(a);
   if (m.nmax == 0 && !m.node_ok) return;      // whole warp beyond the last node (uniform)
 
-  V acc[NV][Kind::NACC];
+  V2 acc[NV][Kind::NACC];
 #pragma unroll
   for (int c = 0; c < NV; ++c)
 #pragma unroll
-    for (int q = 0; q < Kind::NACC; ++q) acc[c][q] = VT<V>::zero();
+    for (int q = 0; q < Kind::NACC; ++q) acc[c][q] = splat2(0.0f);
 
   EdgeRecs<LPN> recs;
   for (int it = 0; it < m.nmax; ++it) {
     const bool valid = (LPN == 32) || (it < m.len);
     const int e = valid ? m.e0 + it : 0;
-#if S7B_COOP_REC
     if (it % LPN == 0) recs.fill(a, m.e0, m.len, it, m.sl);
     const int4 rec = recs.get(it);
-#else
-    const int4 rec = __ldg(a.rec + e);
-#endif
     float Y[Kind::NY];
     load_Y<Kind>(a.Y + (size_t)e * a.ny_stride, Y);
     const float* __restrict__ xrow = a.x + (size_t)rec.x * a.dim_x + role.x_off;
     const float tt = __int_as_float(rec.z);
 #pragma unroll
     for (int c = 0; c < NV; ++c) {
-      const int u = m.uc0 + CH * LPN * c;
-      V x[Kind::D1], w[Kind::NPATH];
+      const int u = m.uc0 + 2 * LPN * c;
+      V2 x[Kind::D1], w[Kind::NPATH];
 #pragma unroll
-      for (int i = 0; i < Kind::D1; ++i) x[i] = VT<V>::load(xrow + i * role.mul + u);
+      for (int i = 0; i < Kind::D1; ++i) x[i] = ldg2(xrow + i * role.mul + u);
 #pragma unroll
       for (int p = 0; p < Kind::NPATH; ++p) {
         if (TABLE) {
-          V a0, a1, a2, a3;
-          VT<V>::coef(a, rec.y, role.w_off[p] + u, a0, a1, a2, a3);
+          V2 a0, a1, a2, a3;
+          table_coef(a, rec.y, role.w_off[p] + u, a0, a1, a2, a3);
           w[p] = fma_(tt, fma_(tt, fma_(tt, a3, a2), a1), a0);
         } else {
-          w[p] = VT<V>::load(a.w + (size_t)e * a.w_numel + role.w_off[p] + u);
+          w[p] = ldg2(a.w + (size_t)e * a.w_numel + role.w_off[p] + u);
         }
-        if (LPN != 32 && !valid) w[p] = VT<V>::zero();
+        if (LPN != 32 && !valid) w[p] = splat2(0.0f);
       }
       Kind::fwd(x, Y, w, acc[c]);
     }
@@ -244,7 +199,10 @@ conv_fwd_kernel(const ConvArgs a, const ConvRole role, float* __restrict__ out) 
         for (int c = 0; c < NV; ++c)
 #pragma unroll
           for (int p = 0; p < Kind::NPATH; ++p)
-            if (Kind::path_l3(p) == l3) mx = fmaxf(mx, VT<V>::amax(acc[c][Kind::acc_off(p) + k]));
+            if (Kind::path_l3(p) == l3) {
+              const V2 v = acc[c][Kind::acc_off(p) + k];
+              mx = fmaxf(mx, fmaxf(fabsf(v.x), fabsf(v.y)));
+            }
 #pragma unroll
         for (int off = LPN / 2; off >= 1; off >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
         if (m.node_ok && m.sl == 0) atomicMax(a.row_max + (size_t)m.n * a.rows_per_node + l3 * l3 + k, __float_as_uint(mx));
@@ -255,12 +213,12 @@ conv_fwd_kernel(const ConvArgs a, const ConvRole role, float* __restrict__ out) 
   float* __restrict__ orow = out + (size_t)m.n * a.dim_mid;
 #pragma unroll
   for (int c = 0; c < NV; ++c) {
-    const int u = m.uc0 + CH * LPN * c;
+    const int u = m.uc0 + 2 * LPN * c;
 #pragma unroll
     for (int p = 0; p < Kind::NPATH; ++p) {
 #pragma unroll
       for (int k = 0; k < 2 * Kind::path_l3(p) + 1; ++k)
-        VT<V>::store(orow + role.out_off[p] + k * role.out_stride[p] + u, acc[c][Kind::acc_off(p) + k]);
+        *reinterpret_cast<float2*>(orow + role.out_off[p] + k * role.out_stride[p] + u) = acc[c][Kind::acc_off(p) + k];
     }
   }
 }
@@ -278,7 +236,7 @@ __global__ void S7B_BWD_BOUNDS
 conv_bwd_kernel(const ConvArgs a, const ConvRole role, const float* __restrict__ gout,
                 float* __restrict__ dx, float* __restrict__ dY_acc, float* __restrict__ dEdr_acc,
                 float* __restrict__ dw) {
-  const LaneMap<NV, LPN, 2> m(a);
+  const LaneMap<NV, LPN> m(a);
   if (m.nmax == 0) return;                    // uniform: no edges in any row of this warp
 
   V2 ga[NV][Kind::NACC];
@@ -305,12 +263,8 @@ conv_bwd_kernel(const ConvArgs a, const ConvRole role, const float* __restrict__
   for (int it = 0; it < m.nmax; ++it) {
     const bool valid = (LPN == 32) || (it < m.len);
     const int e = valid ? m.e0 + it : 0;
-#if S7B_COOP_REC
     if (it % LPN == 0) recs.fill(a, m.e0, m.len, it, m.sl);
     const int4 rec = recs.get(it);
-#else
-    const int4 rec = __ldg(a.rec + e);
-#endif
     float Y[Kind::NY];
     load_Y<Kind>(a.Y + (size_t)e * a.ny_stride, Y);
     const float* __restrict__ xrow = a.x + (size_t)rec.x * a.dim_x + role.x_off;

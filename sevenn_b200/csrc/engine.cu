@@ -161,6 +161,7 @@ struct S7bEngine {
   RadialDesc radial;
   bool radial_ready = false;
   int ny_stride = 8;
+  int max_lx = 0;                         // largest n_lx of any layer = number of per-l1 parts of dY_acc / dEdr_acc
   // graph
   int n_nodes = 0, n_local = 0, n_interior = 0;
   int64_t n_edges = 0;
@@ -350,15 +351,6 @@ __global__ void csr_from_sorted_kernel(const int* __restrict__ centre, const int
   for (int c = max(prev, -1) + 1; c <= min(cur, n_nodes); ++c) rowptr[c] = (int)e;
 }
 
-// out[n, k] = in[k, n]
-__global__ void transpose_kernel(const float* __restrict__ in, float* __restrict__ out, int K, int N) {
-  const size_t total = (size_t)K * N;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-    const int n = (int)(i / K), k = (int)(i - (size_t)n * K);
-    out[i] = in[(size_t)k * N + n];
-  }
-}
-
 // ---- tensor-core linear: host side --------------------------------------------------------------
 // Pre-sliced weights of one block-diagonal linear (see tc_gemm.cuh): per block l the three bf16 slices of
 // W^T in the canonical K-major UMMA layout, cut into (n tile, 32-wide K chunk) blobs that one
@@ -369,6 +361,12 @@ struct TcWeights {
   bool ok = false;
   struct Blk { int K, N, NT; size_t q_off, fb_off; } blk[kMaxL];
 };
+
+// The node linear `name` of layer L runs on the tensor cores: the option is on and its weights were packed.
+static bool tc_ready(const LayerCfg& L, const char* name) {
+  auto it = L.tcw.find(name);
+  return g_opt_tc_gemm && it != L.tcw.end() && it->second && it->second->ok;
+}
 
 // column tiling of an N-wide block: as few tiles of <= 128 columns as possible, tile width a multiple of 16;
 // the last tile may be padded (zero weights, masked in the epilogue)
@@ -615,10 +613,9 @@ static int irreps_linear(const float* A, int lda, const int* a_off, const int* a
 static int node_linear(const LayerCfg& L, const char* name, RowExp& re, bool fresh_re, int n_l_A, const float* A,
                        int lda, const int* a_off, const int* a_K, float* C, int ldc, const int* c_off,
                        const int* c_N, int n_l, const float* W, int n_nodes, bool accumulate, cudaStream_t st) {
-  auto it = L.tcw.find(name);
-  if (g_opt_tc_gemm && it != L.tcw.end() && it->second && it->second->ok) {
+  if (tc_ready(L, name)) {
     if (fresh_re && launch_row_exponents(re, A, lda, a_off, a_K, n_l_A, n_nodes, st)) return 1;
-    return launch_tc_linear(*it->second, re, A, lda, a_off, a_K, C, ldc, c_off, c_N, n_l, n_nodes, accumulate, st);
+    return launch_tc_linear(*L.tcw.at(name), re, A, lda, a_off, a_K, C, ldc, c_off, c_N, n_l, n_nodes, accumulate, st);
   }
   return irreps_linear(A, lda, a_off, a_K, C, ldc, c_off, c_N, n_l, W, n_nodes, accumulate, st);
 }
@@ -643,6 +640,45 @@ static int dense_gemm(const float* A, int K, float* C, int N, const float* W, in
     a.nblocks = 1;
     a.blk[0] = LinBlock{W, 1, K, N, 0, K, 0, N};
     if (launch_gemm(a, st)) return 1;
+  }
+  return 0;
+}
+
+// One tensor-core linear with weights from the host (the test entry points below): packs W_host, computes
+// the row exponents of A, launches, waits for `st` and frees the packed weights and exponents again.
+// `unsupported` is the error when the shapes have no tensor-core form.
+static int tc_linear_once(const float* W_host, const char* unsupported, const float* A, int lda, const int* a_off,
+                          const int* a_K, float* C, int ldc, const int* c_off, const int* c_N, int n_l, int n_nodes,
+                          bool accumulate, cudaStream_t st) {
+  TcWeights w;
+  RowExp re;
+  int rc = tc_build_weights(w, W_host, a_K, c_N, n_l);
+  if (!rc && !w.ok) rc = fail(unsupported);
+  if (!rc) rc = launch_row_exponents(re, A, lda, a_off, a_K, n_l, n_nodes, st);
+  if (!rc) rc = launch_tc_linear(w, re, A, lda, a_off, a_K, C, ldc, c_off, c_N, n_l, n_nodes, accumulate, st);
+  cudaStreamSynchronize(st);
+  w.q.release();
+  w.fb.release();
+  re.buf.release();
+  return rc;
+}
+
+// launch(l1, stream) for every l1 block of layer L, profiled as `label`.t.l1.  With concurrent convolutions
+// (and not profiling) l1 >= 1 run on the side streams, forked from `st` before the first launch and joined
+// back into it after each; otherwise everything runs on `st` in order.
+template <class Launch>
+static int fork_join_l1(S7bEngine* e, const LayerCfg& L, cudaStream_t st, const char* label, int t, Launch launch) {
+  const bool par = e->concurrent && g_opt_concurrent && !e->prof.enabled && L.n_lx > 1;
+  if (par) S7B_CUDA_CHECK(cudaEventRecord(e->ev_fork, st));
+  for (int l1 = 0; l1 < L.n_lx; ++l1) {
+    cudaStream_t s1 = (par && l1 > 0) ? e->side[l1] : st;
+    if (par && l1 > 0) S7B_CUDA_CHECK(cudaStreamWaitEvent(s1, e->ev_fork, 0));
+    ProfScope ps(e->prof, s1, label, t, l1);
+    if (launch(l1, s1)) return 1;
+    if (par && l1 > 0) {
+      S7B_CUDA_CHECK(cudaEventRecord(e->ev_join[l1], s1));
+      S7B_CUDA_CHECK(cudaStreamWaitEvent(st, e->ev_join[l1], 0));
+    }
   }
   return 0;
 }
@@ -712,18 +748,9 @@ int s7b_dense_linear(const float* A, const float* W, float* C, int64_t rows, int
   std::vector<float> hw((size_t)K * N);
   S7B_CUDA_CHECK(cudaMemcpyAsync(hw.data(), W, hw.size() * sizeof(float), cudaMemcpyDeviceToHost, st));
   S7B_CUDA_CHECK(cudaStreamSynchronize(st));
-  TcWeights w;
-  RowExp re;
   const int Ks[1] = {K}, Ns[1] = {N}, zero[1] = {0};
-  int rc = tc_build_weights(w, hw.data(), Ks, Ns, 1);
-  if (!rc && !w.ok) rc = fail("tensor-core weights could not be built");
-  if (!rc) rc = launch_row_exponents(re, A, K, zero, Ks, 1, (int)rows, st);
-  if (!rc) rc = launch_tc_linear(w, re, A, K, zero, Ks, C, N, zero, Ns, 1, (int)rows, false, st);
-  cudaStreamSynchronize(st);
-  w.q.release();
-  w.fb.release();
-  re.buf.release();
-  return rc;
+  return tc_linear_once(hw.data(), "tensor-core weights could not be built", A, K, zero, Ks, C, N, zero, Ns, 1,
+                        (int)rows, false, st);
 }
 
 // Debug: record a timeline of CTA 0 of the NEXT tensor-core linear launches into a device buffer the caller
@@ -750,28 +777,17 @@ int s7b_block_linear(const float* A, int32_t lda, int32_t n_nodes, int32_t n_l, 
   if (!A || !C || !W_host || !a_off || !a_K || !c_off || !c_N) return fail("null argument");
   if (n_l < 1 || n_l > kMaxL || n_nodes < 1) return fail("bad sizes");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (use_tc)
+    return tc_linear_once(W_host, "shapes not supported by the tensor-core linear", A, lda, a_off, a_K, C, ldc, c_off,
+                          c_N, n_l, n_nodes, accumulate != 0, st);
   size_t wn = 0;
   for (int l = 0; l < n_l; ++l) wn += (size_t)a_K[l] * c_N[l];
-  int rc = 0;
-  if (use_tc) {
-    TcWeights w;
-    RowExp re;
-    rc = tc_build_weights(w, W_host, a_K, c_N, n_l);
-    if (!rc && !w.ok) rc = fail("shapes not supported by the tensor-core linear");
-    if (!rc) rc = launch_row_exponents(re, A, lda, a_off, a_K, n_l, n_nodes, st);
-    if (!rc) rc = launch_tc_linear(w, re, A, lda, a_off, a_K, C, ldc, c_off, c_N, n_l, n_nodes, accumulate != 0, st);
-    cudaStreamSynchronize(st);
-    w.q.release();
-    w.fb.release();
-    re.buf.release();
-  } else {
-    float* dW = nullptr;
-    S7B_CUDA_CHECK(cudaMalloc((void**)&dW, wn * sizeof(float)));
-    cudaMemcpy(dW, W_host, wn * sizeof(float), cudaMemcpyHostToDevice);
-    rc = irreps_linear(A, lda, a_off, a_K, C, ldc, c_off, c_N, n_l, dW, n_nodes, accumulate != 0, st);
-    cudaStreamSynchronize(st);
-    cudaFree(dW);
-  }
+  float* dW = nullptr;
+  S7B_CUDA_CHECK(cudaMalloc((void**)&dW, wn * sizeof(float)));
+  cudaMemcpy(dW, W_host, wn * sizeof(float), cudaMemcpyHostToDevice);
+  const int rc = irreps_linear(A, lda, a_off, a_K, C, ldc, c_off, c_N, n_l, dW, n_nodes, accumulate != 0, st);
+  cudaStreamSynchronize(st);
+  cudaFree(dW);
   return rc;
 }
 
@@ -810,6 +826,7 @@ int s7b_engine_create(const S7bModelDesc* d, S7bEngine** out) {
     delete e;
     return fail("the first layer input must be scalars only");
   }
+  for (const LayerCfg& L : e->layers) e->max_lx = std::max(e->max_lx, L.n_lx);
   e->ny_stride = (d->lmax_filter == 3) ? 16 : ((d->lmax_filter == 2) ? 8 : 4);
   const int T = d->n_layers;
   e->x.resize(T);
@@ -953,10 +970,8 @@ int s7b_engine_set_graph(S7bEngine* e, int32_t n_nodes, int32_t n_local, int64_t
   rc |= e->rec.ensure(E * sizeof(int4));
   rc |= e->Y.ensure(E * e->ny_stride * sizeof(float));
   rc |= e->rlen.ensure(E * sizeof(float));
-  int max_lx = 0;
-  for (auto& L : e->layers) max_lx = std::max(max_lx, L.n_lx);
-  rc |= e->dY_acc.ensure((size_t)max_lx * E * e->ny_stride * sizeof(float));
-  rc |= e->dEdr_acc.ensure((size_t)max_lx * E * sizeof(float));
+  rc |= e->dY_acc.ensure((size_t)e->max_lx * E * e->ny_stride * sizeof(float));
+  rc |= e->dEdr_acc.ensure((size_t)e->max_lx * E * sizeof(float));
   rc |= e->fedge.ensure(E * 3 * sizeof(float));
   size_t max_mid = 0, max_h = 0, max_g = 0, max_x = 0, max_W = 0;
   for (int t = 0; t < T; ++t) {
@@ -1063,10 +1078,8 @@ static int run_stage_impl(S7bEngine* e, int stage, int t, void* stream) {
         else if (LF == 2) edge_fwd_kernel<2><<<grd, blk, 0, st>>>(e->radial, e->d_edge_vec, e->d_src, nE, e->ny_stride, e->rec.as<int4>(), e->Y.as<float>(), e->rlen.as<float>(), emb);
         else edge_fwd_kernel<3><<<grd, blk, 0, st>>>(e->radial, e->d_edge_vec, e->d_src, nE, e->ny_stride, e->rec.as<int4>(), e->Y.as<float>(), e->rlen.as<float>(), emb);
         S7B_LAUNCH_CHECK();
-        int max_lx = 0;
-        for (auto& L : e->layers) max_lx = std::max(max_lx, L.n_lx);
-        S7B_CUDA_CHECK(cudaMemsetAsync(e->dY_acc.p, 0, (size_t)max_lx * Ecap * e->ny_stride * sizeof(float), st));
-        S7B_CUDA_CHECK(cudaMemsetAsync(e->dEdr_acc.p, 0, (size_t)max_lx * Ecap * sizeof(float), st));
+        S7B_CUDA_CHECK(cudaMemsetAsync(e->dY_acc.p, 0, (size_t)e->max_lx * Ecap * e->ny_stride * sizeof(float), st));
+        S7B_CUDA_CHECK(cudaMemsetAsync(e->dEdr_acc.p, 0, (size_t)e->max_lx * Ecap * sizeof(float), st));
         if (!table) S7B_CUDA_CHECK(cudaMemsetAsync(e->demb_acc.p, 0, (size_t)E * e->desc.n_basis * sizeof(float), st));
       }
       const LayerCfg& L0 = e->layers[0];
@@ -1109,7 +1122,7 @@ static int run_stage_impl(S7bEngine* e, int stage, int t, void* stream) {
       if (stage == S7B_STAGE_FWD_CONV_INTERIOR) ca.n_dst = e->n_interior;
       if (stage == S7B_STAGE_FWD_LAYER_A2) ca.n_begin = e->n_interior;
       // the convolution kernels also leave the row maxima of `mid` for the tensor-core self_interaction_2
-      const bool fused_rows = g_opt_tc_gemm && L.tcw.count("si2") && L.tcw.at("si2") && L.tcw.at("si2")->ok;
+      const bool fused_rows = tc_ready(L, "si2");
       if (fused_rows) {
         e->re_mid.rows_per_node = L.n_lg * L.n_lg;
         e->re_mid.bits = true;
@@ -1117,20 +1130,10 @@ static int run_stage_impl(S7bEngine* e, int stage, int t, void* stream) {
         ca.row_max = e->re_mid.buf.as<unsigned int>();
         ca.rows_per_node = e->re_mid.rows_per_node;
       }
-      {
-        const bool par = e->concurrent && g_opt_concurrent && !e->prof.enabled && L.n_lx > 1;
-        if (par) S7B_CUDA_CHECK(cudaEventRecord(e->ev_fork, st));
-        for (int l1 = 0; l1 < L.n_lx; ++l1) {
-          cudaStream_t s1 = (par && l1 > 0) ? e->side[l1] : st;
-          if (par && l1 > 0) S7B_CUDA_CHECK(cudaStreamWaitEvent(s1, e->ev_fork, 0));
-          ProfScope ps(e->prof, s1, "conv_fwd", t, l1);
-          if (launch_conv_fwd(l1, LF, L.lmax_out, table, ca, L.roles[l1], e->mid.as<float>(), s1)) return 1;
-          if (par && l1 > 0) {
-            S7B_CUDA_CHECK(cudaEventRecord(e->ev_join[l1], s1));
-            S7B_CUDA_CHECK(cudaStreamWaitEvent(st, e->ev_join[l1], 0));
-          }
-        }
-      }
+      if (fork_join_l1(e, L, st, "conv_fwd", t, [&](int l1, cudaStream_t s1) {
+            return launch_conv_fwd(l1, LF, L.lmax_out, table, ca, L.roles[l1], e->mid.as<float>(), s1);
+          }))
+        return 1;
       if (stage == S7B_STAGE_FWD_CONV_INTERIOR) return 0;
       // self_interaction_2 accumulated onto the self-connection already stored in g[t]
       const float* si2 = lparam(e, t, "si2");
@@ -1141,8 +1144,7 @@ static int run_stage_impl(S7bEngine* e, int stage, int t, void* stream) {
       }
       // gate
       // gate; with the tensor-core linears the kernel also leaves the row exponents of h for self_interaction_1 / sc
-      const bool h_rows = g_opt_tc_gemm && t + 1 < T && e->layers[t + 1].tcw.count("si1") && e->layers[t + 1].tcw.at("si1") &&
-                          e->layers[t + 1].tcw.at("si1")->ok && L.n_lg * L.n_lg <= 16;
+      const bool h_rows = t + 1 < T && tc_ready(e->layers[t + 1], "si1") && L.n_lg * L.n_lg <= 16;
       {
         ProfScope ps(e->prof, st, "gate_fwd", t);
         if (h_rows) {
@@ -1201,7 +1203,7 @@ static int run_stage_impl(S7bEngine* e, int stage, int t, void* stream) {
       if (head && t > 0 && Nn > 0) S7B_CUDA_CHECK(cudaMemsetAsync(e->dx.p, 0, (size_t)Nn * L.dim_x * sizeof(float), st));
       if (Nl == 0) return 0;
       if (head) {
-        const bool dg_rows = g_opt_gate_bwd_rows && g_opt_tc_gemm && L.tcw.count("si2T") && L.tcw.at("si2T") && L.tcw.at("si2T")->ok && L.n_lg * L.n_lg <= 16;
+        const bool dg_rows = g_opt_gate_bwd_rows && tc_ready(L, "si2T") && L.n_lg * L.n_lg <= 16;
         {
           ProfScope ps(e->prof, st, "gate_bwd", t);
           if (dg_rows) {      // ... and the row exponents of dg for si2^T / sc^T
@@ -1224,20 +1226,12 @@ static int run_stage_impl(S7bEngine* e, int stage, int t, void* stream) {
         ConvArgs ca = make_conv_args(e, t, e->x[t].as<float>());
         if (stage == S7B_STAGE_BWD_LAYER_A1) ca.n_begin = e->n_interior;     // boundary atoms first: they own the ghost rows of dx
         if (stage == S7B_STAGE_BWD_LAYER_A2) ca.n_dst = e->n_interior;
-        const bool par = e->concurrent && g_opt_concurrent && !e->prof.enabled && L.n_lx > 1;
-        if (par) S7B_CUDA_CHECK(cudaEventRecord(e->ev_fork, st));
-        for (int l1 = 0; l1 < L.n_lx; ++l1) {
-          float* dY = e->dY_acc.as<float>() + (size_t)l1 * Ecap * e->ny_stride;
-          float* dEdr = e->dEdr_acc.as<float>() + (size_t)l1 * Ecap;
-          cudaStream_t s1 = (par && l1 > 0) ? e->side[l1] : st;
-          if (par && l1 > 0) S7B_CUDA_CHECK(cudaStreamWaitEvent(s1, e->ev_fork, 0));
-          ProfScope ps(e->prof, s1, "conv_bwd", t, l1);
-          if (launch_conv_bwd(l1, LF, L.lmax_out, table, t > 0, ca, L.roles[l1], e->mid.as<float>(), e->dx.as<float>(), dY, dEdr, table ? nullptr : e->dwbuf.as<float>(), s1)) return 1;
-          if (par && l1 > 0) {
-            S7B_CUDA_CHECK(cudaEventRecord(e->ev_join[l1], s1));
-            S7B_CUDA_CHECK(cudaStreamWaitEvent(st, e->ev_join[l1], 0));
-          }
-        }
+        if (fork_join_l1(e, L, st, "conv_bwd", t, [&](int l1, cudaStream_t s1) {
+              float* dY = e->dY_acc.as<float>() + (size_t)l1 * Ecap * e->ny_stride;
+              float* dEdr = e->dEdr_acc.as<float>() + (size_t)l1 * Ecap;
+              return launch_conv_bwd(l1, LF, L.lmax_out, table, t > 0, ca, L.roles[l1], e->mid.as<float>(), e->dx.as<float>(), dY, dEdr, table ? nullptr : e->dwbuf.as<float>(), s1);
+            }))
+          return 1;
         if (!table && tail) {
           // radial MLP backward: dw -> demb (accumulated over layers)
           const float *w0T = lparam(e, t, "mlp0T"), *w1T = lparam(e, t, "mlp1T"), *w2T = lparam(e, t, "mlp2T");
@@ -1280,14 +1274,12 @@ static int run_stage_impl(S7bEngine* e, int stage, int t, void* stream) {
       if (E > 0 && Nl > 0) {
         const int blk = 256;
         const int grd = (int)((Ecap + blk - 1) / blk);
-        int max_lx = 0;
-        for (auto& L : e->layers) max_lx = std::max(max_lx, L.n_lx);
         const float* dEdr = table ? e->dEdr_acc.as<float>() : nullptr;
         const float* demb = table ? nullptr : e->demb_acc.as<float>();
         ProfScope ps(e->prof, st, "edge_bwd_force_scatter");
-        if (LF == 1) edge_bwd_kernel<1><<<grd, blk, 0, st>>>(e->radial, e->d_edge_vec, nE, Ecap, e->ny_stride, max_lx, e->dY_acc.as<float>(), dEdr, demb, e->fedge.as<float>());
-        else if (LF == 2) edge_bwd_kernel<2><<<grd, blk, 0, st>>>(e->radial, e->d_edge_vec, nE, Ecap, e->ny_stride, max_lx, e->dY_acc.as<float>(), dEdr, demb, e->fedge.as<float>());
-        else edge_bwd_kernel<3><<<grd, blk, 0, st>>>(e->radial, e->d_edge_vec, nE, Ecap, e->ny_stride, max_lx, e->dY_acc.as<float>(), dEdr, demb, e->fedge.as<float>());
+        if (LF == 1) edge_bwd_kernel<1><<<grd, blk, 0, st>>>(e->radial, e->d_edge_vec, nE, Ecap, e->ny_stride, e->max_lx, e->dY_acc.as<float>(), dEdr, demb, e->fedge.as<float>());
+        else if (LF == 2) edge_bwd_kernel<2><<<grd, blk, 0, st>>>(e->radial, e->d_edge_vec, nE, Ecap, e->ny_stride, e->max_lx, e->dY_acc.as<float>(), dEdr, demb, e->fedge.as<float>());
+        else edge_bwd_kernel<3><<<grd, blk, 0, st>>>(e->radial, e->d_edge_vec, nE, Ecap, e->ny_stride, e->max_lx, e->dY_acc.as<float>(), dEdr, demb, e->fedge.as<float>());
         S7B_LAUNCH_CHECK();
         force_scatter_kernel<<<(Nl * 32 + blk - 1) / blk, blk, 0, st>>>(e->d_rowptr, e->d_src, e->d_edge_vec, e->fedge.as<float>(), Nl, e->forces.as<float>(), e->virial.as<double>(), av ? e->atomic_virial.as<float>() : nullptr);
         S7B_LAUNCH_CHECK();
